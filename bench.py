@@ -19,6 +19,11 @@ exchange is an NCCL all-gather of one 48-byte VRF candidate per rank per step (S
 
 `--impl reference` times the CPU oracle (the reference's own provider cannot be built here:
 DESIGN.md §3) on rank 0 only.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step of each arm returned to its caller
+(every 8th of its first 2^21 labels and the VRF nonce candidate) as float .npy files, so that two builds can be
+compared output for output on identical inputs.  The sampled label indices are fixed: they depend neither on the
+batch (as long as it holds 2^21 labels) nor on --steps, so a wave size that differs with free HBM or occupancy moves none.
 """
 from __future__ import annotations
 
@@ -41,6 +46,12 @@ NUM_LABELS_4SU = 4 * 2**32
 METRIC = "POST labels/sec (scrypt N=8192 init)"
 ALU_OPS_PER_BLOCKMIX = 553                         # alu-pipe SASS instructions per BlockMix of the shipped kernel (profiles/)
 HBM_FALLBACK_GBS = 6650.0                          # /opt/skills/guides/B200_PROFILING.md fallback
+# Each arm's last step starts at a fixed index of the rank's shard and its earlier steps lie contiguously below it, so
+# consecutive calls continue one another (the engine pre-fills the first layer of the range that follows a call).  The
+# default batch follows the engine's wave size (free HBM, occupancy); anchoring the last step keeps its first labels at
+# the same indices whatever the wave.  Each arm stays inside one 2^32-aligned window for ~780 steps of 5.5 M labels.
+DEV_LAST_START, E2E_LAST_START = 2**33 - 2**26, 2**34 - 2**26
+DUMP_SPAN, DUMP_EVERY = 1 << 21, 8                 # --dump-outputs keeps every 8th label of a step's first 2^21: 2^18 rows
 
 
 def measured_peaks():
@@ -260,6 +271,18 @@ def _timed(fn) -> float:
     return time.perf_counter() - t0
 
 
+def dump_outputs(out_dir: str, arm: str, labels, index, vrf) -> None:
+    """DIR/<arm>_*.npy: sampled labels (uint8[rows, 16] as float32), their label indices and the VRF nonce candidate
+    (index, or -1 when there is none, and its 32-byte label, zeros when there is none) as float64 / float32."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"labels": labels.astype(np.float32), "label_index": index.astype(np.float64),
+              "vrf_index": np.array([vrf[0] if vrf else -1], dtype=np.float64),
+              "vrf_label32": np.frombuffer(vrf[1] if vrf else bytes(32), dtype=np.uint8).astype(np.float32)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{arm}_{name}.npy"), a)
+
+
 def bench_k2pow(b2, provider: int, with_cpu: bool) -> dict:
     """BASELINE.json configs[4] on one GPU: k2pow (RandomX) nonce search over one challenge, difficulty 0 so that nothing
     stops it early; hashes/s over whole device batches (device time from the engine's CUDA events), dataset resident.
@@ -340,7 +363,11 @@ def main() -> None:
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-verify", action="store_true", help="skip the configs[2] verify-batch measurement")
     ap.add_argument("--no-k2pow", action="store_true", help="skip the configs[4] k2pow (RandomX) measurement")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs of each arm to DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        print("bench.py: --dump-outputs ignored: the reference arm times the oracle, which returns no labels",
+              file=sys.stderr)
     if args.warmup < 3:
         args.warmup = 3
 
@@ -381,9 +408,16 @@ def main() -> None:
     d_out = torch.empty((batch, 16), dtype=torch.uint8, device=dev)        # labels stay in HBM for `value`
     h_out = np.empty((batch, 16), dtype=np.uint8)                          # host sink for `e2e`
 
+    # steps: the device-resident arm's warm-up and timed steps, two e2e warm-up steps that continue them, a gap, then
+    # the e2e timed steps
+    dev_last = args.warmup + args.steps - 1
+    e2e_first = 2 * args.warmup + args.steps + 2
+    e2e_last = e2e_first + args.steps - 1
+
     def shard_start(step: int) -> int:
         # weak scaling: every rank initialises its own contiguous slice of a (4*world)-SU space
-        return rank * NUM_LABELS_4SU + step * batch
+        last, last_start = (dev_last, DEV_LAST_START) if step < e2e_first else (e2e_last, E2E_LAST_START)
+        return rank * NUM_LABELS_4SU + last_start + (step - last) * batch
 
     sharding = importlib.import_module("go-spacemesh_b200.sharding")
 
@@ -419,13 +453,14 @@ def main() -> None:
         return el, bracket_ms, calls_ms
 
     debug = bool(os.environ.get("B200POST_BENCH_DEBUG"))
+    last_vrf = {}                                                          # arm -> the VRF candidate of its latest step
 
     def step_dev(s: int):
         t_a = time.perf_counter()
         vrf = b2.labels_range_dev(commitment, N_SCRYPT, shard_start(s), batch, d_out.data_ptr(), provider=local_rank,
                                   vrf_difficulty_=diff)
         t_b = time.perf_counter()
-        exchange(vrf)
+        last_vrf["dev"] = exchange(vrf)
         if debug:
             print(f"[rank {rank}] step {s}: call {1e3 * (t_b - t_a):.1f} ms (device {b2.last_call_ms(local_rank):.1f}), "
                   f"exchange {1e3 * (time.perf_counter() - t_b):.1f} ms", file=sys.stderr, flush=True)
@@ -437,7 +472,7 @@ def main() -> None:
                                             ctypes.cast(ctypes.c_char_p(diff), ctypes.c_void_p), ctypes.byref(nonce), None)
         if rc:
             raise RuntimeError(b2.lib().b200post_last_error().decode())
-        exchange((int(nonce.index), bytes(nonce.label32)) if nonce.found else None)
+        last_vrf["e2e"] = exchange((int(nonce.index), bytes(nonce.label32)) if nonce.found else None)
 
     # ---- device-resident arm (value)
     for w in range(args.warmup):
@@ -451,11 +486,18 @@ def main() -> None:
     clocks = sampler.stop() if rank == 0 else None
     launches = b2.launch_count() - launches0
     romix_ms, romix_k, romix_labels = b2.romix_time(provider=local_rank, reset=True)
+    dump = bool(args.dump_outputs) and rank == 0
+    if dump:            # the same rows of both arms' last steps; they do not depend on the batch once it is >= DUMP_SPAN
+        rows = np.arange(0, min(batch, DUMP_SPAN), DUMP_EVERY)
+        dump_outputs(args.dump_outputs, "dev", d_out[torch.from_numpy(rows).to(dev)].cpu().numpy(),
+                     shard_start(dev_last) + rows, last_vrf["dev"])
 
     # ---- end-to-end arm (host buffers through the reference-facing C-ABI call)
     for w in range(2):
         step_e2e(args.warmup + args.steps + w)
-    wall_e2e, dev_ms_e2e, _ = timed(step_e2e, args.steps, 2 * args.warmup + args.steps + 2)
+    wall_e2e, dev_ms_e2e, _ = timed(step_e2e, args.steps, e2e_first)
+    if dump:
+        dump_outputs(args.dump_outputs, "e2e", h_out[rows], shard_start(e2e_last) + rows, last_vrf["e2e"])
 
     total_labels = batch * args.steps * world
     # device-event time is the clock for `value` (max over ranks); wall clock is the cross-check
